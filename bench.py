@@ -1,6 +1,6 @@
 """bench.py -- real-time factor of the stem-separation hot path (BASELINE.json metric) on N B200s, or the CPU reference arm.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload mdx|htdemucs_ft|mdx23c|vr] [--also htdemucs_ft|none]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload mdx|htdemucs_ft|mdx23c|vr] [--also htdemucs_ft|none] [--dump-outputs DIR]
 
 Workloads (BASELINE.json configs; there are no model files offline, so every network runs seeded synthetic weights of the released
 geometry -- data: "synthetic"):
@@ -158,7 +158,8 @@ class Ctx:
         return t
 
     def timed(self, fn, steps, warmup):
-        """`warmup` untimed + exactly `steps` timed calls, barrier + synchronize on both sides, CUDA events, max over ranks -> ms per step."""
+        """`warmup` untimed + exactly `steps` timed calls, barrier + synchronize on both sides, CUDA events, max over ranks
+        -> (ms per step, what the last timed call returned)."""
         torch = self.torch
         for _ in range(warmup):
             fn()
@@ -166,11 +167,12 @@ class Ctx:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         self.barrier()
         e0.record()
-        for _ in range(steps):
-            fn()
+        for _ in range(steps - 1):
+            fn()  # the result is dropped before the next call, so its memory is reused as in every other step
+        last = fn()
         e1.record()
         self.barrier()
-        return self.max_over_ranks(e0.elapsed_time(e1))[0] / steps
+        return self.max_over_ranks(e0.elapsed_time(e1))[0] / steps, last
 
 
 def music(n, seed):
@@ -181,6 +183,32 @@ def music(n, seed):
 
     base = O.synth_music(min(n, 30 * SR), seed=seed)
     return np.tile(base, (1, -(-n // base.shape[1])))[:, :n].copy()
+
+
+DUMP_BYTES = 60_000_000  # all the files of one --dump-outputs run stay under 64 MB
+
+
+def dump_outputs(out_dir, prefix, arrays, budget):
+    """Write the stems of one timed step as out_dir/<prefix>_<name>.npy (float32) for output-for-output comparison of two builds.
+
+    `arrays`: {name: CUDA float32 tensor with time on the last axis, the same length for all}.  When they do not fit `budget` bytes, every array keeps
+    the same fixed, seeded sample of time positions (sorted); the positions are written as out_dir/<prefix>_sample_index.npy (float64, exact)."""
+    import numpy as np
+    import torch
+
+    if not arrays:  # a VR rank without tracks
+        return
+    lengths = {t.shape[-1] for t in arrays.values()}
+    assert len(lengths) == 1, f"{prefix}: outputs of different lengths {sorted(lengths)}"
+    n = lengths.pop()
+    rows = sum(t.numel() // n for t in arrays.values())
+    k = min(n, budget // (4 * rows + 8))
+    idx = np.sort(np.random.default_rng(0).choice(n, k, replace=False)) if k < n else np.arange(n)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{prefix}_sample_index.npy"), idx.astype(np.float64))
+    idx_d = torch.from_numpy(idx).to(next(iter(arrays.values())).device)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{prefix}_{name}.npy"), t.index_select(-1, idx_d).float().cpu().numpy())
 
 
 # ======================================================================================================== MDX (the headline)
@@ -242,6 +270,10 @@ class MdxWorkload:
 
     def step_device(self):
         return self.eng.separate_device(self.mix_dev, 0.9, 0.0)
+
+    def outputs(self, result):
+        p, s = result  # (N, 2) each
+        return {"primary": p.T, "secondary": s.T}
 
     def step_e2e(self):
         if self.ctx.world > 1:
@@ -383,6 +415,9 @@ class DemucsWorkload:
         part = self.eng.demix_device(self.mix_dev, self.offsets)
         return self.eng.gather(part, self.N)
 
+    def outputs(self, result):
+        return {"sources": result}  # (4, 2, N)
+
     def step_e2e(self):
         self.h2d, self.d2h = self.eng.demix_host(self.mix_host, self.out_host, self.offsets)
 
@@ -466,6 +501,9 @@ class MdxcWorkload:
 
     def step_device(self):
         return self.eng.gather(self.eng.demix_device(self.mix_dev), self.N)
+
+    def outputs(self, result):
+        return {"stems": result}  # (num_targets, 2, N)
 
     def step_e2e(self):
         d = self.mix_host.cuda(non_blocking=True)
@@ -553,10 +591,16 @@ class VrWorkload:
         self.patches = None
 
     def step_device(self):
+        out = []
         for d in self.dev:
             spec = self.eng.loading_mix(d)
             y, v = self.eng.inference(spec)
-            self.eng.spec_to_wav(y), self.eng.spec_to_wav(v)
+            out.append((self.eng.spec_to_wav(y), self.eng.spec_to_wav(v)))
+        return out
+
+    def outputs(self, result):
+        """This rank's tracks: primary and secondary (2, M) of each."""
+        return {f"track{t}_{stem}": w for t, pair in zip(self.mine, result) for stem, w in zip(("primary", "secondary"), pair)}
 
     def step_e2e(self):
         h2d = d2h = 0
@@ -652,8 +696,8 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
-def measure(wl, ctx, args, steps, warmup, with_cpu):
-    """One workload on this rank set -> the JSON line (rank 0) or None."""
+def measure(wl, ctx, args, steps, warmup, with_cpu, dump_bytes=DUMP_BYTES):
+    """One workload on this rank set -> the JSON line (rank 0) or None.  With --dump-outputs, rank 0 writes what the last timed step returned."""
     from audio_separator.separator.b200 import _lib
 
     wl.setup(ctx)
@@ -665,10 +709,13 @@ def measure(wl, ctx, args, steps, warmup, with_cpu):
     if ctx.rank == 0:
         sampler.start()
     launches0 = _lib.launch_count()
-    ms_step = ctx.timed(wl.step_device, steps, 0)
+    ms_step, last = ctx.timed(wl.step_device, steps, 0)
     launches = ctx.sum_over_ranks(_lib.launch_count() - launches0)[0]
     clocks = sampler.summary() if ctx.rank == 0 else None
-    ms_e2e = ctx.timed(wl.step_e2e, steps, 1)
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, wl.name, wl.outputs(last), dump_bytes)
+    del last
+    ms_e2e, _ = ctx.timed(wl.step_e2e, steps, 1)
     h2d, d2h = ctx.sum_over_ranks(wl.h2d, wl.d2h)
     peaks = load_peaks()
     roof = wl.roofline(peaks) if isinstance(wl, MdxWorkload) else wl.roofline(peaks, ms_step)
@@ -703,7 +750,11 @@ def main():
     ap.add_argument("--precision", type=int, default=1)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<workload>_<name>.npy (float32; a fixed seeded sample of time positions, under 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.batch is None:
         args.batch = 8 if args.gpus == 1 else min(12, -(-68 // args.gpus))  # 8 chunks per forward measured 2 % faster than 4 on one box (1242 vs 1215)
     sys.path.insert(0, os.path.join(ROOT, "oracle"))  # synthetic weights + programme material generators, and the cpu legs
@@ -711,8 +762,10 @@ def main():
         return run_reference(args)
     ctx = Ctx(args)
     warmup = max(args.warmup, 3)
-    line = measure(WORKLOADS[args.workload](args), ctx, args, args.steps, warmup, with_cpu=not args.no_cpu_baseline)
-    if args.workload == "mdx" and args.also in WORKLOADS and args.also != "mdx":
+    with_also = args.workload == "mdx" and args.also in WORKLOADS and args.also != "mdx"
+    dump_bytes = DUMP_BYTES // 2 if with_also else DUMP_BYTES
+    line = measure(WORKLOADS[args.workload](args), ctx, args, args.steps, warmup, with_cpu=not args.no_cpu_baseline, dump_bytes=dump_bytes)
+    if with_also:
         import gc
         import signal
 
@@ -729,7 +782,7 @@ def main():
         gc.collect()
         ctx.torch.cuda.empty_cache()
         try:
-            extra = measure(WORKLOADS[args.also](args), ctx, args, min(args.steps, 2), 3, with_cpu=not args.no_cpu_baseline)
+            extra = measure(WORKLOADS[args.also](args), ctx, args, args.steps, 3, with_cpu=not args.no_cpu_baseline, dump_bytes=dump_bytes)
         except Exception as e:  # noqa: BLE001
             import traceback
 
