@@ -370,9 +370,15 @@ int b200sep_gather_pairs_f32(const float* src, const int* idx, float* dst, int64
 int b200sep_mask_average_f32(const float* mask_gathered, const int* csr_offsets, const int* csr_positions, float* mask_out, int64_t rows, int n_gather, int n_out,
                              void* stream);
 /* Roformer branch of MDXCSeparator.demix (mdxc_separator.py:310-343): out[c][q] = sum_i window[q - starts[i]] * chunks[i][c][q - starts[i]] /
- * max(sum_i window[q - starts[i]], 1e-10); chunks (n_chunks, channels, len), starts device int64[n_chunks] */
+ * max(sum_i window[q - starts[i]], 1e-10); chunks (n_chunks, channels, len), starts device int64[n_chunks], non-decreasing */
 int b200sep_overlap_add_starts(const float* chunks, const int64_t* starts, const float* window, int n_chunks, int channels, int len, int64_t n_out, float* out,
                                void* stream);
+/* Time-sharded form: `chunks` (n_local, channels, len) holds the global chunks [first, first + n_local) only, `starts` is the whole global list, and the
+ * samples [q_begin, q_end) of the (channels, n_out) output are written to out[c * out_ld + q - out_base].  Every chunk covering that range must be
+ * local (B200SEP_ERR_ARG otherwise); when the run is not the whole list, checking this reads two entries of `starts` back and synchronises `stream`.
+ * Each sample gets the same contributions in the same order as from b200sep_overlap_add_starts, so a slice is bit-identical to the full call's columns. */
+int b200sep_overlap_add_starts_range(const float* chunks, const int64_t* starts, const float* window, int first, int n_local, int n_chunks, int channels, int len,
+                                     int64_t n_out, int64_t q_begin, int64_t q_end, float* out, int64_t out_ld, int64_t out_base, void* stream);
 
 /* nn.LSTM(bidirectional=True), one layer (LSTMModule of VR 5.1, layers_new.py:124-149): the recurrence only.  x_proj (2, T, N, 4*hid) = the input
  * projections x_t @ W_ih^T + b_ih + b_hh of the forward / reverse direction (gate order i, f, g, o; computed with gemm_f32), w_hh (2, 4*hid, hid);

@@ -5,6 +5,10 @@ ctor `(common_config, arch_config)` with arch keys segment_size / override_model
 pitch_shift, `separate(path, custom_output_names)`, `demix(mix) -> {instrument: (2, N)}`.  The chunk loop runs on the GPU
 through libb200sep.so (MdxcEngine for TFC_TDF_net checkpoints, RoformerEngine for BS-Roformer and Mel-Band Roformer checkpoints -- the Roformer branch of
 demix, mdxc_separator.py:272-343).  Pitch shifting is not part of this path.
+
+arch key `b200_sharded` (default False): one process per GPU in an initialised torch.distributed process group (backend nccl); every rank calls
+separate(path) on the same file, each computes the chunks of its part of the track (b200/sharded.py), rank 0 gathers the stems, writes the files and
+returns their names, the other ranks return [].
 """
 import os
 
@@ -26,12 +30,20 @@ class MDXCSeparator(CommonSeparator):
         self.batch_size = arch_config.get("batch_size", 1)
         self.pitch_shift = arch_config.get("pitch_shift", 0)
         self.process_all_stems = arch_config.get("process_all_stems", True)
+        self.sharded = bool(arch_config.get("b200_sharded", False))
         self.is_roformer = bool(self.is_roformer_model)
         if self.pitch_shift:
             raise NotImplementedError("pitch_shift is not part of the accelerated path")
         if not torch.cuda.is_available():
             raise RuntimeError("MDXCSeparator (B200 build) needs a CUDA device: there is no CPU path in this package")
         self.torch_device = torch.device("cuda", torch.cuda.current_device())
+        self._dist = {}
+        if self.sharded:
+            import torch.distributed as dist
+
+            if not dist.is_initialized():
+                raise RuntimeError("mdxc_params['b200_sharded'] needs an initialised torch.distributed process group (backend nccl, one process per GPU)")
+            self._dist = {"dist": dist}
         self.is_primary_stem_main_target = bool(self.model_data_cfgdict["training"].get("target_instrument"))  # :69, both model families
         self._engines = {}  # dim_t -> engine: the chunk length is fixed per engine, and separate() switches it for clips shorter than 10 s (:137-143)
         self.load_model()
@@ -61,13 +73,13 @@ class MDXCSeparator(CommonSeparator):
         dim_t = int(self.segment_size if self.override_model_segment_size else cfg["inference"]["dim_t"])
         if dim_t not in self._engines:
             if self.is_roformer:
-                eng = RoformerEngine(self.net, dim_t, self.overlap, audio.get("sample_rate", 44100), len(training["instruments"]), max(1, int(self.batch_size)))
+                eng = RoformerEngine(self.net, dim_t, self.overlap, audio.get("sample_rate", 44100), len(training["instruments"]), max(1, int(self.batch_size)), **self._dist)
                 self._engines[dim_t] = (self.net, eng, self.net.forward)
             else:
                 targets = 1 if training.get("target_instrument") else len(training["instruments"])
                 net = TfcNet(self._state, audio["dim_f"], dim_t, model["num_subbands"], audio.get("num_channels", 2), model["num_scales"], model["num_blocks_per_scale"],
                              model["num_channels"], model["growth"], model["bottleneck_factor"], targets, max_batch=max(1, int(self.batch_size)))
-                eng = MdxcEngine(net, audio["n_fft"], audio["hop_length"], audio["dim_f"], dim_t, self.overlap)
+                eng = MdxcEngine(net, audio["n_fft"], audio["hop_length"], audio["dim_f"], dim_t, self.overlap, **self._dist)
                 self._engines[dim_t] = (net, eng, eng.model_run)
         self.net, self.engine, self.model_run = self._engines[dim_t]
 
@@ -90,11 +102,18 @@ class MDXCSeparator(CommonSeparator):
         self.net = BSRoformerNet(rcfg, state, device=self.torch_device)
         self._select_engine()
 
+    def _demix_engine(self, orig):
+        """(S, 2, N) ndarray of the engine's stems; None on the ranks other than 0 of a sharded run (they hold only their slice)."""
+        out = self.engine.gather(self.engine.demix_device(torch.as_tensor(orig).to(self.torch_device)), orig.shape[1])
+        return None if out is None else out.cpu().numpy()
+
     def _demix_roformer(self, mix):
         """Roformer branch of demix + the stem dictionary (mdxc_separator.py:272-343, :406-468)."""
         training = self.model_data_cfgdict["training"]
         orig = np.ascontiguousarray(mix, dtype=np.float32)
-        out = self.engine.demix_device(torch.as_tensor(orig).to(self.torch_device)).cpu().numpy()
+        out = self._demix_engine(orig)
+        if out is None:
+            return None
         if self.net.cfg.num_stems > 1:
             return {k: v for k, v in zip(training["instruments"], out)}
         primary = out[0]
@@ -103,11 +122,13 @@ class MDXCSeparator(CommonSeparator):
         return primary
 
     def demix(self, mix):
-        """(2, N) ndarray -> {instrument: (2, N) ndarray} (mdxc_separator.py:406-434) or the single target's array."""
+        """(2, N) ndarray -> {instrument: (2, N) ndarray} (mdxc_separator.py:406-434) or the single target's array; None on a sharded rank other than 0."""
         if self.is_roformer:
             return self._demix_roformer(mix)
         orig = np.ascontiguousarray(mix, dtype=np.float32)
-        out = self.engine.demix_device(torch.as_tensor(orig).to(self.torch_device)).cpu().numpy()
+        out = self._demix_engine(orig)
+        if out is None:
+            return None
         training = self.model_data_cfgdict["training"]
         if self.net.num_targets > 1:
             return {k: v for k, v in zip(training["instruments"], out)}
@@ -127,6 +148,8 @@ class MDXCSeparator(CommonSeparator):
             self._select_engine()
         mix = normalize(wave=np.array(mix, dtype=np.float32), max_peak=self.normalization_threshold, min_peak=self.amplification_threshold)  # :149
         source = self.demix(mix)
+        if source is None:  # a sharded rank other than 0: rank 0 writes the files
+            return []
         output_files = []
         if isinstance(source, dict):  # (:156-214)
             training = self.model_data_cfgdict["training"]

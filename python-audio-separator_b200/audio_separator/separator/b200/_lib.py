@@ -113,6 +113,7 @@ _SIGS = {
     "b200sep_gather_pairs_f32": (i32, [vp, vp, vp, i64, i32, i32, vp]),
     "b200sep_mask_average_f32": (i32, [vp, vp, vp, vp, i64, i32, i32, vp]),
     "b200sep_overlap_add_starts": (i32, [vp, vp, vp, i32, i32, i32, i64, vp, vp]),
+    "b200sep_overlap_add_starts_range": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, i64, i64, i64, vp, i64, i64, vp]),
     "b200sep_ensemble_f32": (i32, [vp, i32, i64, vp, i32, vp, vp]),
     "b200sep_ensemble_spec_abs": (i32, [vp, i32, i64, i32, i32, vp, vp]),
     "b200sep_selftest_umma_gemm": (i32, [vp, vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, i32, vp]),

@@ -303,9 +303,14 @@ class BSRoformerNet:
 
 
 class RoformerEngine:
-    """Roformer branch of MDXCSeparator.demix (mdxc_separator.py:272-343) with `batch_size` chunks per forward."""
+    """Roformer branch of MDXCSeparator.demix (mdxc_separator.py:272-343) with `batch_size` chunks per forward.
 
-    def __init__(self, net: BSRoformerNet, dim_t: int, overlap, sample_rate=44100, n_instruments=1, batch_size=1):
+    With `dist` (torch.distributed, nccl, one process per GPU) the chunk list is time-sharded (b200/sharded.py, plan_start_shards): rank r finalises the
+    output samples [N*r/W, N*(r+1)/W), computes the chunks that start there and receives from its left neighbour the chunks that reach into its range."""
+
+    def __init__(self, net: BSRoformerNet, dim_t: int, overlap, sample_rate=44100, n_instruments=1, batch_size=1, dist=None, group=None):
+        from .sharded import ShardRunner
+
         self.net = net
         cfg = net.cfg
         self.chunk_size = int(cfg.stft_hop_length) * (int(dim_t) - 1)  # :301
@@ -320,27 +325,56 @@ class RoformerEngine:
         from .graphs import GraphedForward
 
         self.graphed = GraphedForward(self.net.forward)
+        self.runner = ShardRunner(dist, group)
+        self.rank, self.world = self.runner.rank, self.runner.world
 
-    def demix_device(self, mix: torch.Tensor) -> torch.Tensor:
-        """mix (2, N) cuda -> (n_out, 2, N): n_out = num_stems rows for multi-stem models, 1 row for single-target models."""
-        N = mix.shape[1]
-        C, step = self.chunk_size, self.step
+    def chunk_starts(self, N: int) -> list[int]:
+        """The chunk grid of a (2, N) track (:310-315): every `step` samples, the tail clamped to N - chunk (repeated when step < chunk)."""
+        C = self.chunk_size
         if N < C:
             raise NotImplementedError(f"tracks shorter than one chunk ({C} samples) are not covered by the accelerated Roformer path")
-        starts = [i if i + C <= N else N - C for i in range(0, N, step)]
+        return [i if i + C <= N else N - C for i in range(0, N, self.step)]
+
+    def _forward_into(self, mix: torch.Tensor, starts, out: torch.Tensor, slot0: int):
+        """One forward over the chunks mix[:, s : s + chunk] for s in `starts` -> out[slot0 : slot0 + len(starts)] as (S*2, chunk) rows."""
+        C, S, n = self.chunk_size, self.net.cfg.num_stems, len(starts)
+        batch = _new((n, 2, C), mix)
+        for j, s in enumerate(starts):
+            batch[j].copy_(mix[:, s : s + C])
+        y = self.graphed(batch)  # (n, 2, L') or (n, S, 2, L'): CUDA-graph replay of the forward's launch list
+        if y.shape[-1] != C:  # safe_len = min(length, x.shape[-1], window) (:252): hop does not divide the chunk -> zero weight beyond the model output
+            raise NotImplementedError("chunk sizes that are not a multiple of the STFT hop are not covered")
+        out[slot0 : slot0 + n].copy_(y.reshape(n, S * 2, C))
+
+    def demix_device(self, mix: torch.Tensor) -> torch.Tensor:
+        """mix (2, N) cuda -> (n_out, 2, N): n_out = num_stems rows for multi-stem models, 1 row for single-target models.  With `dist`: this rank's
+        (n_out, 2, q1 - q0) slice of it (gather() assembles the whole on rank 0)."""
+        N = mix.shape[1]
+        C = self.chunk_size
+        starts = self.chunk_starts(N)
         S = self.net.cfg.num_stems
-        chunks = _new((len(starts), S * 2, C), mix)
-        for i0 in range(0, len(starts), self.batch_size):
-            group = starts[i0 : i0 + self.batch_size]
-            batch = _new((len(group), 2, C), mix)
-            for j, s in enumerate(group):
-                batch[j].copy_(mix[:, s : s + C])
-            y = self.graphed(batch)  # (g, 2, L') or (g, S, 2, L'): CUDA-graph replay of the forward's launch list
-            Lp = y.shape[-1]
-            if Lp != C:  # safe_len = min(length, x.shape[-1], window) (:252): hop does not divide the chunk -> zero weight beyond the model output
-                raise NotImplementedError("chunk sizes that are not a multiple of the STFT hop are not covered")
-            chunks[i0 : i0 + len(group)].copy_(y.reshape(len(group), S * 2, C))
         sd = torch.tensor(starts, dtype=torch.int64, device=mix.device)
-        out = _new((S * 2, N), mix)
-        check(lib.b200sep_overlap_add_starts(_ptr(chunks), _ptr(sd), _ptr(self.window), len(starts), S * 2, C, N, _ptr(out), _stream()), "overlap_add_starts")
-        return out.view(S, 2, N)
+        if self.runner.dist is None:
+            chunks = _new((len(starts), S * 2, C), mix)
+            for i0 in range(0, len(starts), self.batch_size):
+                self._forward_into(mix, starts[i0 : i0 + self.batch_size], chunks, i0)
+            out = _new((S * 2, N), mix)
+            check(lib.b200sep_overlap_add_starts(_ptr(chunks), _ptr(sd), _ptr(self.window), len(starts), S * 2, C, N, _ptr(out), _stream()), "overlap_add_starts")
+            return out.view(S, 2, N)
+        from .sharded import plan_start_shards
+
+        sh = plan_start_shards(N, self.world, starts, C)[self.rank]
+        local = _new((sh.halo + sh.n_own, S * 2, C), mix)  # [halo | own]
+        self.runner.wait_all(self.runner.run_units(sh, local, lambda buf, slot0, unit0, n: self._forward_into(mix, starts[unit0 : unit0 + n], buf, slot0), self.batch_size))
+        n_q = sh.q1 - sh.q0
+        out = _new((S * 2, n_q), mix)
+        if n_q:
+            check(lib.b200sep_overlap_add_starts_range(_ptr(local), _ptr(sd), _ptr(self.window), sh.c0 - sh.halo, sh.halo + sh.n_own, len(starts), S * 2, C, N, sh.q0, sh.q1,
+                                                       _ptr(out), n_q, sh.q0, _stream()), "overlap_add_starts_range")
+        return out.view(S, 2, n_q)
+
+    def gather(self, part: torch.Tensor, N: int):
+        """Rank 0: the full (S, 2, N) stems from every rank's demix_device slice (None elsewhere); identity on a single GPU."""
+        if self.world == 1:
+            return part
+        return self.runner.gather_cols(part, [(N * r // self.world, N * (r + 1) // self.world) for r in range(self.world)], N)

@@ -1,15 +1,17 @@
 """Time-sharding of ONE track across the GPUs of a box (BASELINE north_star: "chunks shard by time across the 8 GPUs
 with overlap-region halo exchange via NCCL").
 
-The reference has no multi-GPU path (SURVEY.md section 2.1); this is new.  All three chunked architectures have the same
-structure (SURVEY.md section 8e): independent units (MDX chunks, mdx_separator.py:335-348; MDX23C chunks, mdxc_separator.py:361-402;
-Demucs segments, demucs/apply.py:215-250) placed every `stride` samples, coupled only by the overlap-add.  Two planners:
+The reference has no multi-GPU path (SURVEY.md section 2.1); this is new.  The chunked architectures all have the same
+structure (SURVEY.md section 8e): independent units (MDX chunks, mdx_separator.py:335-348; MDX23C and Roformer chunks, mdxc_separator.py:310-402;
+Demucs segments, demucs/apply.py:215-250) placed every `stride` samples, coupled only by the overlap-add.  Three planners:
 
 * `plan_shards`        -- MDX: contiguous chunk ranges, rank r finalises the padded positions [c0*step, c1*step).
 * `plan_range_shards`  -- MDX23C / Demucs: rank r finalises a fixed range [q0, q1) of OUTPUT samples (the same for every pass of a
                           Demucs bag / shift loop, so the accumulation order per sample is the single-GPU order and the result is
                           bit-identical); a unit belongs to the rank its first output sample falls in.
-In both, a rank needs the trailing units of its LEFT neighbour that reach into its range: one `isend`/`irecv` pair between
+* `plan_start_shards`  -- Roformer: the same over an explicit, non-decreasing start list (the tail chunk clamped to N - chunk);
+                          `plan_range_shards` is its stride form.
+In each, a rank needs the trailing units of its LEFT neighbour that reach into its range: one `isend`/`irecv` pair between
 time-neighbours (NCCL p2p over NVLink), posted as soon as those units are computed so the transfer overlaps the remaining forwards.
 The finalised slices go to rank 0 with point-to-point receives straight into the full-size stem buffers, or -- end-to-end entry points --
 every rank copies its own slice into a host buffer shared between the ranks (8 PCIe links in parallel, no gather at all).
@@ -67,11 +69,23 @@ def plan_range_shards(n_out: int, world: int, n_units: int, stride: int, unit_le
     [n_out*r/world, n_out*(r+1)/world) and owns the units whose first output sample (clamped into [0, n_out)) lies in that range."""
     if n_units < 1 or stride < 1 or unit_len < 1:
         raise ValueError("plan_range_shards: bad grid")
+    return plan_start_shards(n_out, world, [i * stride - base for i in range(n_units)], unit_len)
+
+
+def plan_start_shards(n_out: int, world: int, starts, unit_len: int) -> list[Shard]:
+    """plan_range_shards over an explicit, non-decreasing start list (Roformer: the tail chunk is clamped to N - chunk, and with step < chunk several
+    entries repeat it): unit i covers the output samples [starts[i], starts[i] + unit_len)."""
+    from bisect import bisect_left, bisect_right
+
+    starts = [int(s) for s in starts]
+    n_units = len(starts)
+    if n_units < 1 or unit_len < 1 or any(b < a for a, b in zip(starts, starts[1:])):
+        raise ValueError("plan_start_shards: bad grid")
     qs = [n_out * r // world for r in range(world + 1)]
-    u0 = [0] + [min(n_units, max(0, -(-(qs[r] + base) // stride))) for r in range(1, world)] + [n_units]
+    u0 = [0] + [bisect_left(starts, qs[r]) for r in range(1, world)] + [n_units]
     shards = []
     for r in range(world):
-        need_lo = 0 if r == 0 else max(0, (qs[r] + base - unit_len) // stride + 1)
+        need_lo = 0 if r == 0 else bisect_right(starts, qs[r] - unit_len)  # first unit that reaches into [qs[r], ...)
         c0, c1 = u0[r], u0[r + 1]
         halo = max(0, c0 - need_lo) if qs[r + 1] > qs[r] else 0
         if r > 0 and halo > 0 and c0 - halo < u0[r - 1]:

@@ -91,21 +91,33 @@ __global__ void mask_apply_kernel(const float* __restrict__ st, const float* __r
 }
 
 // Roformer branch of MDXCSeparator.demix (mdxc_separator.py:310-343): result += x * window; counter += window; result / clamp(counter, 1e-10)
-// as a gather over the chunks covering each output sample.  chunks (n_chunks, channels, len); chunk i is placed at starts[i].
-__global__ void ola_starts_kernel(const float* __restrict__ chunks, const int64_t* __restrict__ starts, const float* __restrict__ window, int n_chunks, int channels,
-                                  int len, int64_t n_out, float* __restrict__ out) {
+// as a gather over the chunks covering each output sample.  chunks (n_local, channels, len) hold the global chunks [first, first + n_local); chunk i
+// is placed at starts[i] (non-decreasing).  The chunks covering q are the contiguous index run with q - len < starts[i] <= q: two binary searches find
+// it, and it is visited in ascending order, so every sample gets the contributions of a scan over all chunks in the same order.
+__device__ __forceinline__ int upper_bound_i64(const int64_t* __restrict__ a, int n, int64_t v) {  // first index with a[i] > v
+  int lo = 0, hi = n;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (__ldg(&a[mid]) <= v) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo;
+}
+
+__global__ void ola_starts_kernel(const float* __restrict__ chunks, const int64_t* __restrict__ starts, const float* __restrict__ window, int first, int n_local,
+                                  int channels, int len, int64_t q_begin, int64_t q_end, float* __restrict__ out, int64_t out_ld, int64_t out_base) {
   const int c = blockIdx.y;
-  for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < n_out; q += (int64_t)gridDim.x * blockDim.x) {
+  const int64_t* st = starts + first;
+  for (int64_t q = q_begin + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < q_end; q += (int64_t)gridDim.x * blockDim.x) {
     float acc = 0.f, cnt = 0.f;
-    for (int i = 0; i < n_chunks; ++i) {
-      const int64_t r = q - __ldg(&starts[i]);
-      if (r >= 0 && r < len) {
-        const float w = __ldg(&window[r]);
-        acc = fmaf(__ldg(&chunks[((int64_t)i * channels + c) * len + r]), w, acc);
-        cnt += w;
-      }
+    const int i1 = upper_bound_i64(st, n_local, q);
+    for (int i = upper_bound_i64(st, i1, q - len); i < i1; ++i) {
+      const int64_t r = q - __ldg(&st[i]);
+      const float w = __ldg(&window[r]);
+      acc = fmaf(__ldg(&chunks[((int64_t)i * channels + c) * len + r]), w, acc);
+      cnt += w;
     }
-    out[(int64_t)c * n_out + q] = acc / fmaxf(cnt, 1e-10f);
+    out[(int64_t)c * out_ld + (q - out_base)] = acc / fmaxf(cnt, 1e-10f);
   }
 }
 
@@ -205,13 +217,36 @@ extern "C" int b200sep_roformer_mask_apply(const float* stft_tf, const float* ma
   return B200SEP_OK;
 }
 
-extern "C" int b200sep_overlap_add_starts(const float* chunks, const int64_t* starts, const float* window, int n_chunks, int channels, int len, int64_t n_out, float* out,
-                                          void* stream) {
+extern "C" int b200sep_overlap_add_starts_range(const float* chunks, const int64_t* starts, const float* window, int first, int n_local, int n_chunks, int channels,
+                                                int len, int64_t n_out, int64_t q_begin, int64_t q_end, float* out, int64_t out_ld, int64_t out_base, void* stream) {
   B2_CHECK_ARG(chunks && starts && window && out && n_chunks >= 1 && channels >= 1 && len >= 1 && n_out >= 1, "overlap_add_starts: bad argument");
-  dim3 grid((unsigned)std::min<int64_t>(cdiv(n_out, 256), kNumSMs * 8), channels);
-  ola_starts_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(chunks, starts, window, n_chunks, channels, len, n_out, out);
+  B2_CHECK_ARG(0 <= first && n_local >= 1 && (int64_t)first + n_local <= n_chunks, "overlap_add_starts: local chunks [%d, %d) are not a run of the %d chunks", first,
+               first + n_local, n_chunks);
+  B2_CHECK_ARG(0 <= q_begin && q_begin <= q_end && q_end <= n_out, "overlap_add_starts: bad output range");
+  B2_CHECK_ARG(out_base >= 0 && out_base <= q_begin && q_end - out_base <= out_ld, "overlap_add_starts: output slice does not cover [%lld, %lld)", (long long)q_begin,
+               (long long)q_end);
+  if (q_end == q_begin) return B200SEP_OK;
+  if (first > 0 || first + n_local < n_chunks) {
+    // every chunk covering [q_begin, q_end) must be local: the chunk before the run ends at or before q_begin, the one after it starts at or after
+    // q_end.  The start list lives on the device; its two boundary entries are read back (a stream synchronisation, sharded calls only).
+    int64_t edge[2] = {INT64_MIN, INT64_MAX};
+    cudaStream_t s = (cudaStream_t)stream;
+    if (first > 0) B2_CUDA(cudaMemcpyAsync(&edge[0], starts + first - 1, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    if (first + n_local < n_chunks) B2_CUDA(cudaMemcpyAsync(&edge[1], starts + first + n_local, sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    B2_CUDA(cudaStreamSynchronize(s));
+    B2_CHECK_ARG((first == 0 || edge[0] + len <= q_begin) && (first + n_local == n_chunks || edge[1] >= q_end),
+                 "overlap_add_starts: outputs [%lld,%lld) need chunks outside the buffer's [%d,%d) (chunk %d starts at %lld, chunk %d at %lld)", (long long)q_begin,
+                 (long long)q_end, first, first + n_local, first - 1, (long long)edge[0], first + n_local, (long long)edge[1]);
+  }
+  dim3 grid((unsigned)std::min<int64_t>(cdiv(q_end - q_begin, 256), kNumSMs * 8), channels);
+  ola_starts_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(chunks, starts, window, first, n_local, channels, len, q_begin, q_end, out, out_ld, out_base);
   B2_LAUNCHED();
   return B200SEP_OK;
+}
+
+extern "C" int b200sep_overlap_add_starts(const float* chunks, const int64_t* starts, const float* window, int n_chunks, int channels, int len, int64_t n_out, float* out,
+                                          void* stream) {
+  return b200sep_overlap_add_starts_range(chunks, starts, window, 0, n_chunks, n_chunks, channels, len, n_out, 0, n_out, out, n_out, 0, stream);
 }
 
 extern "C" int b200sep_gather_pairs_f32(const float* src, const int* idx, float* dst, int64_t rows, int n_src_pairs, int n_gather, void* stream) {
