@@ -430,6 +430,17 @@ int b200sep_selftest_umma_conv3x3(const float* x, const float* w_host, float* ou
  *            up == 0: out(B,Cout,T/2,F/2) = act(conv2d(x, w(Cout,Cin,2,2), stride=2) * scale + shift);  w is a HOST pointer, skip may be NULL */
 int b200sep_selftest_umma_updown(const float* x, const float* w_host, const float* skip, float* out, int B, int Cin, int Cout, int T, int F,
                                  const float* scale, const float* shift, int relu, int up, void* stream);
+/*   ex     : the epilogue options MDX23C uses.  kind 0 conv3x3, 1 pw (1x1), 2 down (2x2 s2), 3 up (2x2 transposed s2); w_host as above
+ *            ((Cout,Cin,3,3) / (Cout,Cin) / (Cout,Cin,2,2) / (Cin,Cout,2,2)).  y = act(op(x)) (act 0 none, 1 ReLU, 2 GELU); then y += res
+ *            (conv3x3, pw) or y *= res (up); then y *= mul (conv3x3, pw); res and mul are (B, Cout, T', F') and may be NULL.  y goes to channels
+ *            [out_c_off, out_c_off + Cout) of out (B, out_c_total, T', F') (out_c_total 0 = Cout), as a pair, or as plain fp32 when out_f32 != 0 (pw only).
+ *            `out` is read first and split into the pair buffer, so channels outside the slice round-trip. */
+int b200sep_selftest_umma_ex(int kind, const float* x, const float* w_host, const float* res, const float* mul, float* out, int B, int Cin, int Cout,
+                             int T, int F, int act, int out_c_total, int out_c_off, int out_f32, void* stream);
+/*   instnorm_act: out (B, C, P) = act(instance_norm(channels [x_c_off, x_c_off + C) of x (B, x_c_total, P); gamma, beta, eps 1e-5)), act 0 / 1 ReLU / 2 GELU;
+ *            gamma / beta are device pointers, P % 8 == 0 */
+int b200sep_selftest_instnorm_act(const float* x, const float* gamma, const float* beta, float* out, int B, int C, int x_c_total, int x_c_off, int64_t P,
+                                  int act, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------
  * CUDA-graph capture of a launch list issued through this ABI (csrc/api.cu): bracket any sequence of operator calls on `stream`, replay it with

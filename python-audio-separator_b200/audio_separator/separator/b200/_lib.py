@@ -119,6 +119,8 @@ _SIGS = {
     "b200sep_selftest_umma_gemm": (i32, [vp, vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, i32, vp]),
     "b200sep_selftest_umma_conv3x3": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, i32, vp]),
     "b200sep_selftest_umma_updown": (i32, [vp, vp, vp, vp, i32, i32, i32, i32, i32, vp, vp, i32, i32, vp]),
+    "b200sep_selftest_umma_ex": (i32, [i32, vp, vp, vp, vp, vp] + [i32] * 9 + [vp]),
+    "b200sep_selftest_instnorm_act": (i32, [vp, vp, vp, vp, i32, i32, i32, i32, i64, i32, vp]),
     "b200sep_capture_begin": (i32, [vp]),
     "b200sep_capture_end": (i32, [vp, vp]),
     "b200sep_graph_launch": (i32, [vp, vp]),

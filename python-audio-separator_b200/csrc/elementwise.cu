@@ -4,6 +4,8 @@
 
 #include <cuda_bf16.h>
 
+#include "umma_ops.cuh"  // split_pair / join_pair (self-test)
+
 namespace b200sep {
 
 using bf16 = __nv_bfloat16;
@@ -137,3 +139,25 @@ int cws_merge_f32(const float* x, float* spec, int B, int S, int Cc, int T, int 
 }
 
 }  // namespace b200sep
+
+// ---------------------------------------------------------------------------------------------------------
+// self-test entry point (C ABI): fp32 in -> split -> instnorm_act_pair -> join -> fp32 out, synchronous
+using namespace b200sep;
+
+extern "C" int b200sep_selftest_instnorm_act(const float* x, const float* gamma, const float* beta, float* out, int B, int C, int x_c_total, int x_c_off, int64_t P,
+                                             int act, void* stream) {
+  B2_CHECK_ARG(x && gamma && beta && out, "selftest_instnorm_act: NULL argument");
+  B2_CHECK_ARG(x_c_off >= 0 && x_c_off + C <= x_c_total && act >= 0 && act <= 2, "selftest_instnorm_act: channels [%d, %d) of %d / act=%d", x_c_off, x_c_off + C,
+               x_c_total, act);
+  cudaStream_t st = (cudaStream_t)stream;
+  uint16_t *x_p = nullptr, *y_p = nullptr;
+  const int64_t nx = (int64_t)B * x_c_total * P, ny = (int64_t)B * C * P;
+  B2_CUDA(cudaMalloc(&x_p, nx * 4));
+  B2_CUDA(cudaMalloc(&y_p, ny * 4));
+  int rc = split_pair(x, x_p, x_p + nx, nx, st);
+  if (!rc) rc = instnorm_act_pair(x_p, x_p + nx, x_c_total, x_c_off, gamma, beta, act, y_p, y_p + ny, B, C, P, st);
+  if (!rc) rc = join_pair(y_p, y_p + ny, out, ny, st);
+  cudaStreamSynchronize(st);
+  cudaFree(x_p); cudaFree(y_p);
+  return rc;
+}

@@ -331,6 +331,11 @@ extern "C" int b200sep_tfcnet_create(b200sep_tfcnet** out, const b200sep_tfcnet_
   B2_CHECK_ARG(cfg->dim_f % cfg->num_subbands == 0 && Fs % (1 << n) == 0 && cfg->dim_t % (1 << n) == 0, "tfcnet_create: dim_f/num_subbands=%d and dim_t=%d must be divisible by 2^%d", Fs,
                cfg->dim_t, n);
   B2_CHECK_ARG(((Fs >> n) % cfg->bn) == 0 && (Fs >> n) % 8 == 0, "tfcnet_create: innermost frequency size %d must be a multiple of 8 and of bn", Fs >> n);
+  // the instance norm of the TDF hidden layer works on planes of (T >> i) * ((Fs >> i) / bn) elements in groups of 8; the bottleneck's is the smallest
+  // (every larger scale's is 4x the next one's)
+  B2_CHECK_ARG((int64_t)(cfg->dim_t >> n) * ((Fs >> n) / cfg->bn) % 8 == 0,
+               "tfcnet_create: the bottleneck's TDF hidden plane (dim_t>>%d) * ((dim_f/num_subbands>>%d)/bn) = %d * %d must be a multiple of 8", n, n, cfg->dim_t >> n,
+               (Fs >> n) / cfg->bn);
   const int64_t expect = b200sep_tfcnet_param_count(cfg);
   B2_CHECK_ARG(expect == n_params, "tfcnet_create: expected %lld parameters for this config, got %lld", (long long)expect, (long long)n_params);
   int devs = 0;

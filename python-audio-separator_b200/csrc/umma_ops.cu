@@ -1387,3 +1387,73 @@ extern "C" int b200sep_selftest_umma_updown(const float* x, const float* w_host,
   if (s_p) cudaFree(s_p);
   return rc;
 }
+
+// Every epilogue option of the conv modes as MDX23C uses them (tfc_net.cu): act, residual (multiplied for UP), multiplier, output channel slice, fp32 store.
+// `out` is split into the pair buffer before the run and joined back after it, so the channels outside the slice must come back unchanged.
+extern "C" int b200sep_selftest_umma_ex(int kind, const float* x, const float* w_host, const float* res, const float* mul, float* out, int B, int Cin, int Cout,
+                                        int T, int F, int act, int out_c_total, int out_c_off, int out_f32, void* stream) {
+  B2_CHECK_ARG(x && w_host && out, "selftest_umma_ex: NULL argument");
+  B2_CHECK_ARG(kind >= 0 && kind <= 3 && act >= 0 && act <= 2 && B >= 1 && T >= 1, "selftest_umma_ex: bad kind=%d / act=%d / B=%d / T=%d", kind, act, B, T);
+  const int ct = out_c_total > 0 ? out_c_total : Cout;
+  B2_CHECK_ARG(out_c_off >= 0 && out_c_off + Cout <= ct, "selftest_umma_ex: channels [%d, %d) do not fit in %d", out_c_off, out_c_off + Cout, ct);
+  B2_CHECK_ARG(!mul || kind <= 1, "selftest_umma_ex: the multiplier exists for conv3x3 and pw only");
+  B2_CHECK_ARG(!res || kind != 2, "selftest_umma_ex: the down conv has no residual");
+  B2_CHECK_ARG(!out_f32 || kind == 1, "selftest_umma_ex: the fp32 store exists for pw only");
+  int kc = 0, n_c = 0, To = T, Fo = F;
+  std::vector<uint16_t> hi, lo;
+  if (kind == 0) {
+    B2_CHECK_ARG(umma_conv_supported(Cin, Cout, F, 3, 3), "selftest_umma_ex: conv3x3 Cin=%d Cout=%d F=%d not supported by the tensor-core path", Cin, Cout, F);
+    umma_conv_choose(Cin, Cout, &kc, &n_c);
+    umma_conv_block_weights(w_host, Cout, Cin, kc, n_c, hi, lo);
+  } else if (kind == 1) {
+    B2_CHECK_ARG(umma_pw_supported(Cin, Cout, F), "selftest_umma_ex: pw Cin=%d Cout=%d F=%d not supported by the tensor-core path", Cin, Cout, F);
+    umma_pw_choose(Cin, Cout, &kc, &n_c);
+    umma_pw_block_weights(w_host, Cout, Cin, kc, n_c, hi, lo);
+  } else {
+    const int up = kind == 3;
+    B2_CHECK_ARG(umma_updown_supported(Cin, Cout, F, up) && (up || T % 2 == 0), "selftest_umma_ex: %s Cin=%d Cout=%d T=%d F=%d not supported by the tensor-core path",
+                 up ? "up" : "down", Cin, Cout, T, F);
+    umma_updown_choose(Cin, Cout, up, &kc, &n_c);
+    if (up) umma_up_block_weights(w_host, Cin, Cout, kc, n_c, hi, lo);
+    else umma_down_block_weights(w_host, Cout, Cin, kc, n_c, hi, lo);
+    To = up ? 2 * T : T / 2;
+    Fo = up ? 2 * F : F / 2;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  uint16_t *x_p = nullptr, *o_p = nullptr, *w_p = nullptr, *r_p = nullptr, *m_p = nullptr;
+  const int64_t nx = (int64_t)B * Cin * T * F, no = (int64_t)B * ct * To * Fo, nr = (int64_t)B * Cout * To * Fo, nw = (int64_t)hi.size();
+  B2_CUDA(cudaMalloc(&x_p, nx * 4));
+  B2_CUDA(cudaMalloc(&w_p, nw * 4));
+  if (!out_f32) B2_CUDA(cudaMalloc(&o_p, no * 4));
+  if (res) B2_CUDA(cudaMalloc(&r_p, nr * 4));
+  if (mul) B2_CUDA(cudaMalloc(&m_p, nr * 4));
+  B2_CUDA(cudaMemcpy(w_p, hi.data(), nw * 2, cudaMemcpyHostToDevice));
+  B2_CUDA(cudaMemcpy(w_p + nw, lo.data(), nw * 2, cudaMemcpyHostToDevice));
+  int rc = split_pair(x, x_p, x_p + nx, nx, st);
+  if (!rc && o_p) rc = split_pair(out, o_p, o_p + no, no, st);
+  if (!rc && r_p) rc = split_pair(res, r_p, r_p + nr, nr, st);
+  if (!rc && m_p) rc = split_pair(mul, m_p, m_p + nr, nr, st);
+  UmmaConvPlan pl;
+  if (!rc) rc = umma_conv_plan_create(&pl, x_p, x_p + nx, B, Cin, T, F, kc);
+  UmmaEpilogue e;
+  e.act = act;
+  if (o_p) { e.out_hi = o_p; e.out_lo = o_p + no; }
+  else e.out_f32 = out;
+  if (r_p) { e.res_hi = r_p; e.res_lo = r_p + nr; }
+  if (m_p) { e.mul_hi = m_p; e.mul_lo = m_p + nr; }
+  e.out_c_total = ct;
+  e.out_c_off = out_c_off;
+  if (!rc) {
+    if (kind == 0) rc = umma_conv_run_ex(pl, w_p, w_p + nw, B, Cout, n_c, e, st);
+    else if (kind == 1) rc = umma_pw_run_ex(pl, w_p, w_p + nw, B, Cout, n_c, e, st);
+    else if (kind == 2) rc = umma_down_run_ex(pl, w_p, w_p + nw, B, Cout, n_c, e, st);
+    else rc = umma_up_run_ex(pl, w_p, w_p + nw, B, Cout, n_c, e, st);
+  }
+  if (!rc && o_p) rc = join_pair(o_p, o_p + no, out, no, st);
+  cudaStreamSynchronize(st);
+  cudaFree(x_p); cudaFree(w_p);
+  if (o_p) cudaFree(o_p);
+  if (r_p) cudaFree(r_p);
+  if (m_p) cudaFree(m_p);
+  return rc;
+}
